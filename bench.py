@@ -2,13 +2,17 @@
 """Benchmark of the DDSP synthesis hot path (BASELINE.json metric: audio Msamples/s at 44.1 kHz,
 128 harmonics; % of the HBM roofline).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload sins|...]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload sins|...] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE).  A "step" is one pass of the
 Sins synthesis path (frame phase scan -> sinusoid bank -> impulse responses -> two time-varying
 FIRs + mix, in-kernel Philox noise) over one batch of B=32 utterances x 10 s per GPU
 (BASELINE configs[1]; configs[3] at N=8 = 256 utterances); at N>1 the step also gathers every
 rank's `signal` to rank 0 over NCCL (the path's only collective).  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR (one GPU) writes what the last timed step returned as DIR/<name>.npy in float32, so that two builds
+can be compared output for output: inputs are seeded and the in-kernel noise seeds come from torch's CPU generator,
+seeded before the first step, so the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -24,6 +28,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 SR, P = 44100, 512
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs: at most this many bytes of .npy files in all
 OTHER_WORKLOADS = ("sins_cfg1", "combsub", "superfast", "combsubfast", "sinegen", "srcmod", "mel", "maskmul")
 
 # N -> (gather mode, chunks, compute streams) chosen by `--gather auto` (measured on B200, see DESIGN.md section 5)
@@ -355,13 +360,24 @@ class Runner:
             return self.stft.get_mel(audio)
         return self.frontend.mask_apply_(audio, self.mask_d[lo:lo + audio.shape[0]], P)
 
+    keep_outputs = False               # step() keeps what the caller receives in self.outputs (--dump-outputs)
+
     def step(self, f0=None):
         if self.w["kind"] in ("mel", "maskmul"):
-            return self._wave_op(self.audio_d)
-        f0 = self.f0_d if f0 is None else f0
-        if self.sg:
-            return self.model(f0[..., 0], P, rand_ini=self.rand_ini, utterance_offset=self.rank * self.B)
-        return self.model(None, f0, None, utterance_offset=self.rank * self.B)[0]
+            out = self._wave_op(self.audio_d)
+        else:
+            f0 = self.f0_d if f0 is None else f0
+            if self.sg:
+                out = self.model(f0[..., 0], P, rand_ini=self.rand_ini, utterance_offset=self.rank * self.B)
+            else:
+                signal, _, (harmonic, noise) = self.model(None, f0, None, utterance_offset=self.rank * self.B)
+                if self.keep_outputs:  # CombSubFast / CombSubSuperFast return the signal three times
+                    self.outputs = ({"signal": signal, "harmonic": harmonic, "noise": noise}
+                                    if self.w["kind"] in ("sins", "combsub") else {"signal": signal})
+                return signal
+        if self.keep_outputs:
+            self.outputs = {"out": out}
+        return out
 
     # rows [lo, hi) of the local batch (for the chunked synth+gather pipeline) -> [hi-lo, row_len]
     @property
@@ -461,6 +477,22 @@ class Runner:
                                                                buf[0].data_ptr(), 0, ir_n.data_ptr(), ir_n.shape[2],
                                                                buf[1].data_ptr(), 0, 1, 0, B, nF, P, st),
                 "ltv_fir_harmonic_1022": lambda: ops.ltv_fir(comb, ir_h, P)}
+
+
+def dump_outputs(outputs, out_dir, torch):
+    """Write each output tensor as out_dir/<name>.npy in float32.  When all of them together exceed DUMP_BYTES, each is
+    replaced by the same fixed, seeded sample of its flattened elements (sorted positions, an equal share of the
+    budget per tensor)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(4 * t.numel() for t in outputs.values())
+    cap = (DUMP_BYTES - 4096) // (4 * len(outputs))
+    for name, t in outputs.items():
+        t = t.detach()
+        if total > DUMP_BYTES and t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), size=cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def time_e2e(run, chunks, flush, reps, torch):
@@ -607,8 +639,14 @@ def main():
     ap.add_argument("--sinegen-impl", default="auto", choices=["auto", "v1", "v2", "v2p", "v2r7"],
                     help="A/B switch for the SineGen / source-module kernel (ops.set_sinegen_impl)")
     ap.add_argument("--breakdown", action="store_true", help="also print per-kernel times to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32; a fixed, "
+                         "seeded sample of each output when all of them exceed 64 MB); one GPU only")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
+    if args.dump_outputs and (args.impl == "reference" or args.e2e_only or args.gpus > 1
+                              or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs the device-timed steps of a single-GPU run")
     if args.impl == "reference":
         return run_reference_arm(args, w)
     args.warmup = max(args.warmup, 3)
@@ -628,7 +666,9 @@ def main():
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
 
+    torch.manual_seed(0)                       # in-kernel noise seeds and SineGen phases: the same on every run
     run = Runner(w, dev, rank, torch)
+    run.keep_outputs = bool(args.dump_outputs)
     e2e_chunks = int(args.e2e_chunks) if args.e2e_chunks.isdigit() else tuple(int(x) for x in args.e2e_chunks.split(","))
     run.e2e_streams = args.e2e_streams
     if args.sinegen_impl != "auto":
@@ -736,6 +776,9 @@ def main():
         wall = time.perf_counter() - wall0
         launches = ops.launches() - n0
         dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+        if args.dump_outputs:
+            dump_outputs(run.outputs, args.dump_outputs, torch)
+            run.keep_outputs, run.outputs = False, None
         gather_checked = check_gather() if do_gather else None
 
         # ---- end to end through the public module API with HOST buffers ----

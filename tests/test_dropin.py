@@ -1,16 +1,23 @@
 """Drop-in contract: constructor arguments, buffers / state-dict keys and class dispatch match
-the reference (SURVEY.md appendix D).  The parts that need the live reference (Unit2Control,
-strict state-dict round trip, patch_reference) run only where /root/reference exists."""
-import contextlib
-import io
+the reference (SURVEY.md appendix D).  The reference's state-dict layouts (keys, shapes, buffers) are stored in
+tests/golden/ref_state_dicts.npz (made by tests/golden/make_golden_models.py from its classes)."""
 import sys
+import types
 
 import pytest
 import torch
 
 import ddsp_svc_b200 as pkg
 from ddsp_svc_b200 import dropin
-from oracle import ref_loader
+from tests import util
+
+# name -> constructor, given the module holding the classes (this package, or the reference's ddsp.vocoder)
+STATE_DICT_CASES = {
+    "Sins": lambda V: V.Sins(44100, 512, 128, 256, 256, n_unit=768, n_spk=1),
+    "CombSub": lambda V: V.CombSub(44100, 512, 256, 512, 256, n_unit=768, n_spk=2),
+    "CombSubSuperFast": lambda V: V.CombSubSuperFast(44100, 512, 2048, n_unit=768, n_spk=1),
+    "CombSubFast": lambda V: V.CombSubFast(44100, 512, n_unit=768, n_spk=1),
+}
 
 
 def test_buffers_and_forward_signature_without_reference():
@@ -50,44 +57,67 @@ def test_module_refuses_cpu_tensors():
         m(None, torch.zeros(1, 3, 1), None)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="live reference not present")
+def _reference_state_dict(module, gold, prefix):
+    """seeded weights in the reference's layout, with the reference's own buffers"""
+    sd = util.seeded_state_dict(module, 0)
+    for k in sd:
+        if prefix + "buffer__" + k in gold:
+            sd[k] = torch.from_numpy(gold[prefix + "buffer__" + k])
+    return sd
+
+
 def test_state_dict_round_trip_with_the_reference_classes(tmp_path):
-    with contextlib.redirect_stdout(io.StringIO()):
-        V, _, RefSineGen = ref_loader.load()
-        cases = [
-            (V.Sins(44100, 512, 128, 256, 256, n_unit=768, n_spk=1), lambda: pkg.Sins(44100, 512, 128, 256, 256, n_unit=768, n_spk=1)),
-            (V.CombSub(44100, 512, 256, 512, 256, n_unit=768, n_spk=2), lambda: pkg.CombSub(44100, 512, 256, 512, 256, n_unit=768, n_spk=2)),
-            (V.CombSubSuperFast(44100, 512, 2048, n_unit=768, n_spk=1), lambda: pkg.CombSubSuperFast(44100, 512, 2048, n_unit=768, n_spk=1)),
-            (V.CombSubFast(44100, 512, n_unit=768, n_spk=1), lambda: pkg.CombSubFast(44100, 512, n_unit=768, n_spk=1)),
-        ]
-        for ref_model, make in cases:
-            ours = make()                                   # uses the reference's Unit2Control
-            sd = ref_model.state_dict()
-            assert list(ours.state_dict().keys()) == list(sd.keys())
-            ours.load_state_dict(sd)                        # strict, like ddsp/vocoder.py:527
-            for k, v in ours.state_dict().items():
-                assert torch.equal(v, sd[k]), k
-        # load_model: config.yaml next to the checkpoint -> class dispatch -> strict load
-        import yaml
-        cfg = {"data": {"sampling_rate": 44100, "block_size": 512, "encoder_out_channels": 768},
-               "model": {"type": "CombSubSuperFast", "win_length": 2048, "n_spk": 1}}
-        (tmp_path / "config.yaml").write_text(yaml.safe_dump(cfg))
-        torch.save({"global_step": 1, "model": cases[2][0].state_dict()}, tmp_path / "model_1.pt")
-        model, args = dropin.load_model(str(tmp_path / "model_1.pt"), device="cpu")
-        assert isinstance(model, pkg.CombSubSuperFast) and args.model.win_length == 2048
-        # patch / unpatch
-        saved = pkg.patch_reference()
-        try:
-            assert V.Sins is pkg.Sins and V.CombSubSuperFast is pkg.CombSubSuperFast
-            assert V.CombSubFast is pkg.CombSubFast
-            import nsf_hifigan.models as nsf
-            assert nsf.SineGen is pkg.SineGen and nsf.SourceModuleHnNSF is pkg.SourceModuleHnNSF
-            model2, _ = V.load_model(str(tmp_path / "model_1.pt"), device="cpu")   # the REFERENCE's loader
-            assert isinstance(model2, pkg.CombSubSuperFast)
-        finally:
-            pkg.unpatch_reference(saved)
-        assert V.Sins is not pkg.Sins and nsf.SourceModuleHnNSF is not pkg.SourceModuleHnNSF
-        ref_sm = nsf.SourceModuleHnNSF(44100, harmonic_num=8)          # state dict of the reference class loads strictly
-        ours_sm = pkg.SourceModuleHnNSF(44100, harmonic_num=8)
-        assert list(ours_sm.state_dict()) == list(ref_sm.state_dict())
-        ours_sm.load_state_dict(ref_sm.state_dict())
+    gold = util.load_golden("ref_state_dicts")
+    for name, make in STATE_DICT_CASES.items():
+        ours = make(pkg)                                # this package's Unit2Control
+        util.check_state_dict_layout(ours, gold, name + "__")
+        sd = _reference_state_dict(ours, gold, name + "__")
+        ours.load_state_dict(sd)                        # strict, like ddsp/vocoder.py:527
+        for k, v in ours.state_dict().items():
+            assert torch.equal(v, sd[k]), k
+    # load_model: config.yaml next to the checkpoint -> class dispatch -> strict load
+    import yaml
+    cfg = {"data": {"sampling_rate": 44100, "block_size": 512, "encoder_out_channels": 768},
+           "model": {"type": "CombSubSuperFast", "win_length": 2048, "n_spk": 1}}
+    (tmp_path / "config.yaml").write_text(yaml.safe_dump(cfg))
+    sd = _reference_state_dict(STATE_DICT_CASES["CombSubSuperFast"](pkg), gold, "CombSubSuperFast__")
+    torch.save({"global_step": 1, "model": sd}, tmp_path / "model_1.pt")
+    model, args = dropin.load_model(str(tmp_path / "model_1.pt"), device="cpu")
+    assert isinstance(model, pkg.CombSubSuperFast) and args.model.win_length == 2048
+    ours_sm = pkg.SourceModuleHnNSF(44100, harmonic_num=8)      # state dict of the reference class loads strictly
+    util.check_state_dict_layout(ours_sm, gold, "SourceModuleHnNSF__")
+    ours_sm.load_state_dict(util.seeded_state_dict(ours_sm, 0))
+
+
+def test_patch_reference_rebinds_and_restores_the_reference_names(monkeypatch):
+    """patch_reference() on modules laid out like the reference's ddsp.vocoder / nsf_hifigan.models / nsf_hifigan.nvSTFT:
+    the reference's entry points resolve these names at call time, so after patching they build this package's
+    classes; unpatch_reference() restores the originals."""
+    mods = {}
+    for modname, names in (("ddsp.vocoder", ("Sins", "CombSub", "CombSubSuperFast", "CombSubFast", "Volume_Extractor")),
+                           ("nsf_hifigan.models", ("SineGen", "SourceModuleHnNSF")), ("nsf_hifigan.nvSTFT", ("STFT",))):
+        m = mods[modname] = types.ModuleType(modname)
+        for n in names:
+            setattr(m, n, type(n, (), {}))
+    for pkgname in ("ddsp", "nsf_hifigan"):
+        parent = types.ModuleType(pkgname)
+        parent.__path__ = []
+        monkeypatch.setitem(sys.modules, pkgname, parent)
+    for modname, m in mods.items():
+        monkeypatch.setitem(sys.modules, modname, m)
+        setattr(sys.modules[modname.split(".")[0]], modname.split(".")[1], m)
+    V, nsf, stft = mods["ddsp.vocoder"], mods["nsf_hifigan.models"], mods["nsf_hifigan.nvSTFT"]
+    originals = {n: getattr(V, n) for n in ("Sins", "CombSub", "CombSubSuperFast", "CombSubFast", "Volume_Extractor")}
+    originals.update(SineGen=nsf.SineGen, SourceModuleHnNSF=nsf.SourceModuleHnNSF)
+    orig_stft = stft.STFT
+    from ddsp_svc_b200 import frontend, mel
+    saved = pkg.patch_reference()
+    try:
+        assert "_not_patched" not in saved
+        assert V.Sins is pkg.Sins and V.CombSub is pkg.CombSub and V.CombSubSuperFast is pkg.CombSubSuperFast
+        assert V.CombSubFast is pkg.CombSubFast and V.Volume_Extractor is frontend.Volume_Extractor
+        assert nsf.SineGen is pkg.SineGen and nsf.SourceModuleHnNSF is pkg.SourceModuleHnNSF and stft.STFT is mel.STFT
+    finally:
+        pkg.unpatch_reference(saved)
+    assert all(getattr(V if hasattr(V, n) else nsf, n) is c for n, c in originals.items())
+    assert stft.STFT is orig_stft

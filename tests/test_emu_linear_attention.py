@@ -56,18 +56,21 @@ def test_matches_fp64_formula(emu, B, H, T, J):
     assert np.abs(out - want).max() < 2e-5 * max(1.0, np.abs(want).max())
 
 
-def test_matches_the_reference_function():
-    """the fp64 formula above IS the reference's linear_attention (pcmer.py:220-229), checked with its own code where present"""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("reference sources not present")
-    ref_loader.load()
-    import ddsp.pcmer as ref_pcmer
+def reference_inputs():
     g = torch.Generator().manual_seed(1)
     q = torch.rand(2, 3, 20, 266, generator=g, dtype=torch.float64)
     k = torch.rand(2, 3, 20, 266, generator=g, dtype=torch.float64)
     v = torch.randn(2, 3, 20, 64, generator=g, dtype=torch.float64)
-    want = ref_pcmer.linear_attention(q, k, v).numpy()
-    ctx = np.einsum("bhtj,bhtd->bhjd", k.numpy(), v.numpy())
-    mine = np.einsum("bhtj,bhjd->bhtd", q.numpy(), ctx) / (np.einsum("bhtj,bhj->bht", q.numpy(), k.numpy().sum(2)) + 1e-8)[..., None]
-    assert np.abs(mine - want).max() < 1e-12
+    return q, k, v
+
+
+def test_matches_the_reference_function():
+    """the fp64 formula above IS the reference's linear_attention (pcmer.py:220-229): checked against its own outputs,
+    stored in tests/golden/ref_oracle_fresh.npz by tests/golden/make_golden_models.py"""
+    from tests import util
+    q, k, v = (t.numpy() for t in reference_inputs())
+    want = util.load_golden("ref_oracle_fresh")["linear_attention"]
+    ctx = np.einsum("bhtj,bhtd->bhjd", k, v)
+    mine = np.einsum("bhtj,bhjd->bhtd", q, ctx) / (np.einsum("bhtj,bhj->bht", q, k.sum(2)) + 1e-8)[..., None]
+    assert want.dtype == np.float64
+    assert np.abs(util.sampled(mine, want.size) - want).max() < 1e-12

@@ -1,56 +1,34 @@
-"""Acceptance run on the GPU: the reference's OWN call (main.py:259, `model(seg_units, seg_f0, seg_volume, spk_id=...,
-spk_mix_dict=...)` under torch.no_grad, then `seg_output *= mask` in place, main.py:260) executed twice on the same
-device -- once with the unmodified reference classes under eager PyTorch, once after `patch_reference()` through the
-reference's own `load_model` (which then builds this package's synthesizers AND its Unit2Control, loaded strictly from
-the reference's checkpoint) -- real torch.split views of dense_out, real spk_id embedding / spk_mix_dict -- and the
-waveforms compared.
+"""Acceptance run on the GPU: the reference's call (main.py:259, `model(seg_units, seg_f0, seg_volume, spk_id=...,
+spk_mix_dict=...)` under torch.no_grad, then `seg_output *= mask` in place, main.py:260) on this package's synthesizers,
+built through `load_model` (config.yaml next to the checkpoint -> class dispatch -> strict load of a checkpoint in the
+reference's layout, this package's Unit2Control included) -- real torch.split views of dense_out, real spk_id embedding
+/ spk_mix_dict -- and the waveforms compared with the reference's classes run on the same seeded weights and inputs.
 
-Needs the reference sources: the live checkout in the build container or the staged copy baseline/_ref/
-(tools/stage_reference.py, travels to the GPU box); skipped when neither exists.
-
-The white noise of the reference comes from torch's CUDA generator (rand_like / randn_like): the test records the tensor
-the reference drew and feeds the same samples to the B200 module (`noise=`), so the full signal is comparable; the exact
-main.py call without `noise=` (in-kernel Philox) is checked on its deterministic part and on the noise level."""
-import contextlib
-import io
-
+The reference's outputs are stored in tests/golden/ref_acceptance.npz (a seeded sample of each waveform plus its full
+RMS; made by tests/golden/make_golden_models.py on the CPU).  Its white noise (rand_like / randn_like) was replaced by
+seeded draws there (tests.util.seeded_draw); the test feeds the same samples to the B200 module (`noise=`), so the full
+signal is comparable; the exact main.py call without `noise=` (in-kernel Philox) is checked on its deterministic part
+and on the noise level."""
+import numpy as np
 import pytest
 import torch
 import yaml
 
 import ddsp_svc_b200 as pkg
-from oracle import ref_loader
 from tests import report, util
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="reference sources not present")]
+pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 SR, P, NU = 44100, 512, 768
-# The reference runs its DSP with CUDA operators here, the kernels follow the reference's CPU path (the oracle, SURVEY
-# A.10): torch's fp32 cumsum accumulates in fp32 on CUDA and in fp64 on the CPU (all-pass phase, SuperFast / SineGen frame
-# scans), so reference-on-GPU differs from reference-on-CPU by a few 1e-6 absolute at this signal level (RMS 0.06-0.08,
-# i.e. <= 1e-4 relative; measured: Sins 5.8e-6, CombSub 6.3e-6, CombSubFast 9e-7, CombSubSuperFast 2.2e-5).  The bound is
-# the north star's 1e-4 RMS; parity at the 1e-8 level is pinned on identical controls by the golden tests.
+SEED = 1
+# The reference's DSP runs on the CPU (the oracle path, SURVEY A.10) and so do the kernels' formulas; reference-on-GPU
+# differs from reference-on-CPU by a few 1e-6 absolute at this signal level (RMS 0.06-0.08, i.e. <= 1e-4 relative:
+# torch's fp32 cumsum accumulates in fp32 on CUDA and in fp64 on the CPU).  The bound is the north star's 1e-4 RMS;
+# parity at the 1e-8 level is pinned on identical controls by the golden tests.
 GATE_RMS = 1e-4
 
 
-@contextlib.contextmanager
-def _record_noise(store):
-    """record what torch.rand_like / torch.randn_like return while the reference runs"""
-    r0, n0 = torch.rand_like, torch.randn_like
-
-    def rand_like(*a, **k):
-        t = r0(*a, **k); store.append(("rand", t)); return t
-
-    def randn_like(*a, **k):
-        t = n0(*a, **k); store.append(("randn", t)); return t
-
-    torch.rand_like, torch.randn_like = rand_like, randn_like
-    try:
-        yield
-    finally:
-        torch.rand_like, torch.randn_like = r0, n0
-
-
+# `make` takes the module holding the classes: ddsp_svc_b200 here, the reference's ddsp.vocoder for the stored outputs
 CASES = {
     "Sins": dict(model={"type": "Sins", "n_harmonics": 128, "n_mag_allpass": 256, "n_mag_noise": 256, "n_spk": 2},
                  make=lambda V: V.Sins(SR, P, 128, 256, 256, n_unit=NU, n_spk=2), uniform=True, parts=True),
@@ -64,114 +42,89 @@ CASES = {
 }
 
 
+def inputs():
+    """one main.py segment (~1.5 s), B = 1, on the CPU: units, f0, volume and the caller's silence mask"""
+    nF = 130
+    g = torch.Generator().manual_seed(2)
+    units = torch.randn(1, nF, NU, generator=g)
+    f0 = 220.0 * 2 ** (torch.rand(1, nF, 1, generator=g) * 0.3)
+    f0[:, 40:48] = 0.0                              # an unvoiced stretch, as f0 extractors produce
+    volume = 0.1 * torch.rand(1, nF, 1, generator=g)
+    mask = (torch.rand(1, nF * P, generator=g) > 0.1).float()
+    return units, f0, volume, mask
+
+
+def calls():
+    spk_id = torch.LongTensor([[2]])
+    return [dict(spk_id=spk_id, spk_mix_dict=None), dict(spk_id=spk_id, spk_mix_dict={1: 0.3, 2: 0.7})]
+
+
+def source_module_f0():
+    f0 = 200.0 + 50.0 * torch.rand(2, 40, generator=torch.Generator().manual_seed(3))
+    f0[:, 10:14] = 0.0
+    return f0
+
+
 @pytest.mark.parametrize("kind", list(CASES))
 def test_main_py_call_reference_vs_patched(kind, tmp_path):
     case = CASES[kind]
-    with contextlib.redirect_stdout(io.StringIO()):
-        V = ref_loader.load()[0]
-        torch.manual_seed(1)
-        ref_model = case["make"](V).to(DEV).eval()
-    nF = 130                                        # one main.py segment (~1.5 s), B = 1
-    g = torch.Generator().manual_seed(2)
-    units = torch.randn(1, nF, NU, generator=g).to(DEV)
-    f0 = (220.0 * 2 ** (torch.rand(1, nF, 1, generator=g) * 0.3)).to(DEV)
-    f0[:, 40:48] = 0.0                              # an unvoiced stretch, as f0 extractors produce
-    volume = (0.1 * torch.rand(1, nF, 1, generator=g)).to(DEV)
-    mask = (torch.rand(1, nF * P, generator=g) > 0.1).float().to(DEV)
-    spk_id = torch.LongTensor([[2]]).to(DEV)
-    calls = [dict(spk_id=spk_id, spk_mix_dict=None), dict(spk_id=spk_id, spk_mix_dict={1: 0.3, 2: 0.7})]
-
+    gold = util.load_golden("ref_acceptance")
     cfg = {"data": {"sampling_rate": SR, "block_size": P, "encoder_out_channels": NU}, "model": case["model"]}
     (tmp_path / "config.yaml").write_text(yaml.safe_dump(cfg))
-    torch.save({"global_step": 1, "model": ref_model.state_dict()}, tmp_path / "model_1.pt")
-
-    refs = []
-    # the reference's control network runs cuDNN convolutions, which use TF32 by default (1e-3 relative): compare against its
-    # true fp32 result
-    tf32 = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
+    torch.save({"global_step": 1, "model": util.seeded_state_dict(case["make"](pkg), SEED)}, tmp_path / "model_1.pt")
+    model, args = pkg.load_model(str(tmp_path / "model_1.pt"), device=DEV)
+    assert type(model) is getattr(pkg, kind)
+    units, f0, volume, mask = (t.to(DEV) for t in inputs())
+    tol = case.get("tol", GATE_RMS)
     with torch.no_grad():
-        for kw in calls:
-            drawn = []
-            with _record_noise(drawn):
-                seg_output, hidden, (s_h, s_n) = ref_model(units, f0, volume, **kw)       # main.py:259, reference classes
-            assert len(drawn) == 1
-            noise = drawn[0][1] * 2 - 1 if case["uniform"] else drawn[0][1]
-            assert (drawn[0][0] == "rand") == case["uniform"]
-            refs.append((seg_output.clone(), hidden.clone(), s_h.clone(), s_n.clone(), noise.reshape(1, -1).clone()))
-
-    torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = tf32
-    saved = pkg.patch_reference()
-    try:
-        with contextlib.redirect_stdout(io.StringIO()):
-            model, args = V.load_model(str(tmp_path / "model_1.pt"), device=DEV)          # the REFERENCE's loader
-        assert isinstance(model, getattr(pkg, kind)) and not isinstance(model, type(ref_model))
-        with torch.no_grad():
-            for kw, (r_sig, r_hid, r_h, r_n, noise) in zip(calls, refs):
-                # (1) same noise samples -> the whole signal is comparable
-                sig, hidden, (s_h, s_n) = model(units, f0, volume, noise=noise, **kw)
-                # this package's Unit2Control (fused kernels + fp32 library GEMMs) against the reference's class in fp32
-                assert util.rms((hidden - r_hid).cpu()) < 1e-4 * max(util.rms(r_hid.cpu()), 1e-6)
-                tol = case.get("tol", GATE_RMS)
-                e = util.rms((sig - r_sig).cpu())
-                report.record("acceptance/%s/%s" % (kind, "mix" if kw["spk_mix_dict"] else "spk"), err=e,
-                              max=(sig - r_sig).abs().max().item(), signal_rms=util.rms(r_sig.cpu()))
-                assert e < tol
-                if case["parts"]:
-                    assert util.rms((s_h - r_h).cpu()) < tol and util.rms((s_n - r_n).cpu()) < tol
-                # (2) the exact main.py lines: no `noise=`, then the in-place mask multiply on the returned tensor
-                seg_output, _, (s_h2, s_n2) = model(units, f0, volume, **kw)
-                if case["parts"]:
-                    assert util.rms((s_h2 - r_h).cpu()) < tol                               # deterministic part
-                    lvl = util.rms(s_n2.cpu()) / max(util.rms(r_n.cpu()), 1e-12)
-                    assert 0.9 < lvl < 1.1                                                 # same noise level, other samples
-                    keep_h = s_h2.clone()
-                else:
-                    lvl = util.rms(seg_output.cpu()) / max(util.rms(r_sig.cpu()), 1e-12)
-                    assert 0.8 < lvl < 1.25
-                before = seg_output.clone()
-                seg_output *= mask                                                          # main.py:260
-                assert torch.equal(seg_output, before * mask)
-                if case["parts"]:
-                    assert torch.equal(s_h2, keep_h)                                       # outputs are not aliased
-    finally:
-        pkg.unpatch_reference(saved)
+        for i, kw in enumerate(calls()):
+            p = "%s__c%d__" % (kind, i)
+            kw = {k: (v.to(DEV) if torch.is_tensor(v) else v) for k, v in kw.items()}
+            drawn = util.stored_draws(gold, p)
+            assert len(drawn) == 1 and (drawn[0][0] == "rand") == case["uniform"]
+            noise = (drawn[0][1] * 2 - 1 if case["uniform"] else drawn[0][1]).reshape(1, -1).to(DEV)
+            r_sig, r_hid, r_h, r_n = (gold.get(p + k) for k in ("signal", "hidden", "harmonic", "noise"))
+            # (1) same noise samples -> the whole signal is comparable
+            sig, hidden, (s_h, s_n) = model(units, f0, volume, noise=noise, **kw)
+            # this package's Unit2Control (fused kernels + fp32 library GEMMs) against the reference's class in fp32
+            assert util.rms(util.sampled(hidden, r_hid.size) - r_hid) < 1e-4 * max(util.rms(r_hid), 1e-6)
+            d = util.sampled(sig, r_sig.size) - r_sig
+            e = util.rms(d)
+            report.record("acceptance/%s/%s" % (kind, "mix" if kw["spk_mix_dict"] else "spk"), err=e,
+                          max=np.abs(d).max(), signal_rms=float(gold[p + "signal_rms"]))
+            assert e < tol
+            if case["parts"]:
+                assert util.rms(util.sampled(s_h, r_h.size) - r_h) < tol and util.rms(util.sampled(s_n, r_n.size) - r_n) < tol
+            # (2) the exact main.py lines: no `noise=`, then the in-place mask multiply on the returned tensor
+            seg_output, _, (s_h2, s_n2) = model(units, f0, volume, **kw)
+            if case["parts"]:
+                assert util.rms(util.sampled(s_h2, r_h.size) - r_h) < tol                    # deterministic part
+                lvl = util.rms(s_n2.cpu()) / max(float(gold[p + "noise_rms"]), 1e-12)
+                assert 0.9 < lvl < 1.1                                                     # same noise level, other samples
+                keep_h = s_h2.clone()
+            else:
+                lvl = util.rms(seg_output.cpu()) / max(float(gold[p + "signal_rms"]), 1e-12)
+                assert 0.8 < lvl < 1.25
+            before = seg_output.clone()
+            seg_output *= mask                                                              # main.py:260
+            assert torch.equal(seg_output, before * mask)
+            if case["parts"]:
+                assert torch.equal(s_h2, keep_h)                                           # outputs are not aliased
 
 
 def test_enhancer_source_module_through_patch_reference():
-    """enhancer.py's generator builds `SourceModuleHnNSF(...)` from nsf_hifigan.models: after patch_reference() that name
-    is the fused B200 module; same state dict, and with the reference's random phases / noise fed in, the same output."""
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref_loader.load()
-    import nsf_hifigan.models as nsf
-    torch.manual_seed(3)
-    ref_sm = nsf.SourceModuleHnNSF(SR, harmonic_num=8).to(DEV).eval()
-    f0 = (200.0 + 50.0 * torch.rand(2, 40)).to(DEV)
-    f0[:, 10:14] = 0.0
-    upp = 512
-    r0 = torch.rand
-    ini = []
-
-    def rec_rand(*a, **k):
-        t = r0(*a, **k); ini.append(t); return t
-
-    drawn = []
-    torch.rand = rec_rand
-    try:
-        with torch.no_grad(), _record_noise(drawn):
-            ref_out = ref_sm(f0, upp)
-    finally:
-        torch.rand = r0
-    rand_ini = ini[0].clone(); rand_ini[..., 0] = 0
-    saved = pkg.patch_reference()
-    try:
-        ours = nsf.SourceModuleHnNSF(SR, harmonic_num=8).to(DEV).eval()
-        assert isinstance(ours, pkg.SourceModuleHnNSF)
-        ours.load_state_dict(ref_sm.state_dict())
-        with torch.no_grad():
-            out = ours(f0, upp, rand_ini=rand_ini, noise=drawn[0][1])
-    finally:
-        pkg.unpatch_reference(saved)
-    e = util.rms((out - ref_out).cpu())
-    report.record("acceptance/source_module", err=e, rms=util.rms(ref_out.cpu()))
-    assert out.shape == ref_out.shape and e < 1e-4      # the reference's fp32 cumsum on CUDA differs from its CPU path
+    """enhancer.py's generator builds `SourceModuleHnNSF(...)` from nsf_hifigan.models, which patch_reference() rebinds to
+    the fused B200 module (tests/test_dropin.py): same state dict, and with the reference's random phases / noise fed in,
+    the same output as the reference's class."""
+    gold = util.load_golden("ref_acceptance")
+    ours = pkg.SourceModuleHnNSF(SR, harmonic_num=8).to(DEV).eval()
+    ours.load_state_dict(util.seeded_state_dict(ours, SEED))
+    drawn = util.stored_draws(gold, "source_module__")
+    assert [k for k, _ in drawn] == ["rand", "randn"]          # SineGen's initial phases, then its additive noise
+    rand_ini = drawn[0][1].clone(); rand_ini[..., 0] = 0
+    with torch.no_grad():
+        out = ours(source_module_f0().to(DEV), 512, rand_ini=rand_ini.to(DEV), noise=drawn[1][1].to(DEV))
+    want = gold["source_module__out"]
+    e = util.rms(util.sampled(out, want.size) - want)
+    report.record("acceptance/source_module", err=e, rms=util.rms(want))
+    assert list(out.shape) == list(gold["source_module__shape"]) and e < 1e-4

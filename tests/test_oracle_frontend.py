@@ -1,6 +1,6 @@
 """The numpy restatement of the caller-side prologue / epilogue (oracle/frontend.py) against outputs of the live
-reference: the committed fixtures tests/golden/frontend_*.npz (made by tests/golden/make_golden_frontend.py) and,
-where the reference is present, its own code executed on fresh inputs."""
+reference: the committed fixtures tests/golden/frontend_*.npz (made by tests/golden/make_golden_frontend.py) and its
+own code's outputs on fresh inputs (tests/golden/ref_oracle_fresh.npz, made by tests/golden/make_golden_models.py)."""
 import glob
 import os
 
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 from oracle import frontend as fe
-from oracle import ref_loader
+from tests import util
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = sorted(glob.glob(os.path.join(HERE, "golden", "frontend_*.npz")))
@@ -29,20 +29,28 @@ def test_restatement_reproduces_the_reference_fixtures(path):
     assert np.array_equal(out, z["fade_out"])
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="live reference not present")
+FRESH = ((11, 9000, 512), (12, 777, 256), (13, 30011, 441))       # (seed, samples, hop)
+FADE_IDX = (0, 1, 250, 399)
+
+
+def fade_inputs(seed):
+    g = np.random.default_rng(seed)
+    return g.standard_normal(400).astype(np.float32), g.standard_normal(500).astype(np.float32)
+
+
 def test_restatement_equals_the_live_reference_on_fresh_inputs():
-    from tests.golden.make_golden_frontend import inputs, reference_function, reference_mask_lines
-    V = ref_loader.load()[0]
-    cf = reference_function("main.py", "cross_fade")
-    for seed, T, hop in ((11, 9000, 512), (12, 777, 256), (13, 30011, 441)):
+    from tests.golden.make_golden_frontend import inputs
+    gold = util.load_golden("ref_oracle_fresh")
+    for seed, T, hop in FRESH:
         audio = inputs(seed, T)
-        want = V.Volume_Extractor(hop).extract(audio)
-        assert np.array_equal(fe.volume_extract(audio, hop), want)
-        assert np.array_equal(fe.volume_mask(want, -45), reference_mask_lines(want, -45))
-        g = np.random.default_rng(seed)
-        a, b = g.standard_normal(400).astype(np.float32), g.standard_normal(500).astype(np.float32)
-        for idx in (0, 1, 250, 399):
-            assert np.array_equal(fe.cross_fade(a, b, idx), cf(a, b, idx))
+        want = gold["fe%d__volume" % seed]
+        vol = fe.volume_extract(audio, hop)
+        assert vol.dtype == want.dtype and np.array_equal(vol, want)
+        assert np.array_equal(fe.volume_mask(want, -45), gold["fe%d__mask" % seed])
+        a, b = fade_inputs(seed)
+        for idx in FADE_IDX:
+            got, want = fe.cross_fade(a, b, idx), gold["fe%d__fade%d" % (seed, idx)]
+            assert got.size == gold["fe%d__fade%d_len" % (seed, idx)] and np.array_equal(util.sampled(got, want.size), want)
 
 
 def test_interpolation_weight_arithmetic_of_the_mask_kernel_equals_torch():

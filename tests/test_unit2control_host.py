@@ -1,19 +1,36 @@
 """Host logic of ddsp_svc_b200.unit2control.Unit2Control on the CPU: parameter tree (state-dict keys / shapes), weight
 packing (k = 3 convolution as one GEMM over shifted inputs, fused q/k/v weights, weight-norm) and the order of operations,
-with the five fused CUDA kernels replaced by their torch definitions, against the reference's class.  (The kernels
-themselves are checked on the GPU in tests/test_gpu_unit2control.py.)  Needs the reference sources."""
-import contextlib
-import io
+with the five fused CUDA kernels replaced by their torch definitions, against the reference's class: its state-dict
+layout and its outputs on seeded weights and inputs, stored in tests/golden/ref_u2c_host.npz by
+tests/golden/make_golden_models.py.  (The kernels themselves are checked on the GPU in tests/test_gpu_unit2control.py.)"""
 import math
 
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
 from ddsp_svc_b200 import unit2control as U
-from oracle import ref_loader
+from tests import util
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference sources not present")
+SEED = 3
+VARIANTS = {"pcmer": (dict(), {"a": 33, "b": 7}),
+            "naive_conformer": (dict(use_naive_v2=True, use_conv_stack=True, use_pitch_aug=True), {"a": 33, "b": 7}),
+            "pcmer_norm_plainconv": (dict(pcmer_norm=True, use_conv_stack=False), {"a": 33, "b": 7})}
+
+
+def inputs():
+    g = torch.Generator().manual_seed(1)
+    units, f0 = torch.randn(2, 50, 64, generator=g), 200 + 100 * torch.rand(2, 50, 1, generator=g)
+    ph, vo = torch.rand(2, 50, 1, generator=g), torch.rand(2, 50, 1, generator=g)
+    return units, f0, ph, vo
+
+
+def calls(kw):
+    c = [dict(spk_id=torch.LongTensor([[2], [3]])), dict(spk_id=torch.LongTensor([[1]]), spk_mix_dict={1: 0.3, 2: 0.7})]
+    if kw.get("use_pitch_aug"):
+        c.append(dict(spk_id=torch.LongTensor([[1], [1]]), aug_shift=torch.tensor([[[2.0]], [[-3.0]]])))
+    return c
 
 
 def _layernorm(x, w, b):
@@ -96,32 +113,20 @@ def torch_kernels(monkeypatch):
     monkeypatch.setattr(U.Unit2Control, "gemm_precision", "fp32")       # plain [O, K] weights in the packed dict
 
 
-@pytest.mark.parametrize("kw", [dict(), dict(use_naive_v2=True, use_conv_stack=True, use_pitch_aug=True),
-                                dict(pcmer_norm=True, use_conv_stack=False)], ids=["pcmer", "naive_conformer", "pcmer_norm_plainconv"])
-def test_parameter_tree_and_host_logic_match_the_reference(kw, torch_kernels):
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref_loader.load()
-    from ddsp.unit2control import Unit2Control as Ref
-    import ddsp.pcmer as ref_pcmer
-    ref_pcmer.FLAG_PCMER_NORM = False
-    torch.manual_seed(3)
-    splits = {"a": 33, "b": 7}
-    ref = Ref(64, 3, splits, **kw).eval()
+@pytest.mark.parametrize("name", list(VARIANTS))
+def test_parameter_tree_and_host_logic_match_the_reference(name, torch_kernels):
+    kw, splits = VARIANTS[name]
+    gold = util.load_golden("ref_u2c_host")
+    torch.manual_seed(SEED)
     ours = U.Unit2Control(64, 3, splits, **kw).eval()
-    assert list(ours.state_dict().keys()) == list(ref.state_dict().keys())
-    assert all(ours.state_dict()[k].shape == v.shape for k, v in ref.state_dict().items())
-    ours.load_state_dict(ref.state_dict())                        # strict
-    g = torch.Generator().manual_seed(1)
-    units, f0 = torch.randn(2, 50, 64, generator=g), 200 + 100 * torch.rand(2, 50, 1, generator=g)
-    ph, vo = torch.rand(2, 50, 1, generator=g), torch.rand(2, 50, 1, generator=g)
-    calls = [dict(spk_id=torch.LongTensor([[2], [3]])), dict(spk_id=torch.LongTensor([[1]]), spk_mix_dict={1: 0.3, 2: 0.7})]
-    if kw.get("use_pitch_aug"):
-        calls.append(dict(spk_id=torch.LongTensor([[1], [1]]), aug_shift=torch.tensor([[[2.0]], [[-3.0]]])))
-    for c in calls:
+    util.check_state_dict_layout(ours, gold, name + "__")
+    ours.load_state_dict(util.seeded_state_dict(ours, SEED))     # strict
+    units, f0, ph, vo = inputs()
+    for i, c in enumerate(calls(kw)):
         with torch.no_grad():
-            wc, wh = ref(units, f0, ph, vo, **c)
             gc, gh = ours(units, f0, ph, vo, **c)
-        dw, dg = torch.cat(list(wc.values()), -1), torch.cat(list(gc.values()), -1)
-        assert (dw - dg).abs().max().item() < 2e-5 * max(1.0, dw.abs().max().item())
-        assert (wh - gh).abs().max().item() < 2e-5 * max(1.0, wh.abs().max().item())
-    ref_pcmer.FLAG_PCMER_NORM = False
+        assert list(gc) == [str(k) for k in gold[name + "__ctrl_names"]]
+        dw, wh = gold["%s__c%d__controls" % (name, i)], gold["%s__c%d__hidden" % (name, i)]
+        dg = util.sampled(torch.cat(list(gc.values()), -1), dw.size)
+        assert np.abs(dw - dg).max() < 2e-5 * max(1.0, np.abs(dw).max())
+        assert np.abs(wh - util.sampled(gh, wh.size)).max() < 2e-5 * max(1.0, np.abs(wh).max())
