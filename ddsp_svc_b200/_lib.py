@@ -95,6 +95,10 @@ SIGNATURES = {
     "b2d_superfast_synth": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_f32p, ctypes.c_int64, c_f32p,
                                            ctypes.c_uint64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                            ctypes.c_int, c_f32p, c_stream]),
+    "b2d_superfast_backward": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_f32p, ctypes.c_int64, c_f32p,
+                                              ctypes.c_uint64, ctypes.c_int64, c_f32p, ctypes.c_int, ctypes.c_int,
+                                              ctypes.c_int, ctypes.c_int, c_f32p, c_f32p, c_f32p, c_f32p,
+                                              ctypes.c_int64, c_stream]),
 }
 
 _lock = threading.Lock()

@@ -205,6 +205,77 @@ __device__ __forceinline__ float4 normals4(unsigned long long seed, unsigned lon
     return make_float4(m1 * c1, m1 * s1, m2 * c2, m2 * s2);
 }
 
+// periodic Hann (first half, win[i] = win[2048 - i]) and the pass twiddles of fft2048
+__device__ __forceinline__ void init_tables(float* winh, float2* tw2, float2* tw3, int tid) {
+    for (int i = tid; i <= kHalf; i += kThreads) winh[i] = 0.5f - 0.5f * cospif((float)i * (2.0f / kN));
+    for (int i = tid; i < 15 * 16; i += kThreads) {
+        const int r = i / 16 + 1, k = i % 16;
+        float sn, cs; sincospif(-2.0f * (float)(r * k) / 256.0f, &sn, &cs);
+        tw2[i] = make_float2(cs, sn);
+    }
+    for (int i = tid; i < 256; i += kThreads) {
+        float sn, cs; sincospif(-2.0f * (float)i / 2048.0f, &sn, &cs);
+        tw3[i] = make_float2(cs, sn);
+    }
+}
+
+__device__ __forceinline__ float win_of(const float* winh, int i) { return winh[i <= kHalf ? i : kN - i]; }
+
+// iSTFT envelope OLA(win^2) over the frames q = 0..nF that exist, at sample i (0 <= i < 512) of hop h
+__device__ __forceinline__ float ola_env(const float* winh, int h, int i, int nF) {
+    float env = 0.f;
+#pragma unroll
+    for (int d = -1; d <= 2; ++d) {
+        const int qq = h + d;
+        if (qq >= 0 && qq <= nF) { const float w = win_of(winh, i - d * kHop + kHalf); env = fmaf(w, w, env); }
+    }
+    return env;
+}
+
+// un-windowed source (comb, noise) of absolute positions [mstart + i_lo, mstart + i_hi) -> src ring slots
+// (i + off) & 2047; positions outside [0, T) follow the STFT's padding (reflect, or zeros when T <= 1024)
+__device__ __forceinline__ void fill_source(float2* src, const float4* __restrict__ fpar, const float* noise_row,
+                                            unsigned long long seed, unsigned long long utt, int T, int P,
+                                            int mstart, int off, int i_lo, int i_hi, int tid) {
+    const float fP = (float)P;
+    const bool reflect = T > kHalf;                              // pad_mode (:672-675)
+#pragma unroll 1
+    for (int i0 = i_lo + (tid << 2); i0 < i_hi; i0 += kThreads << 2) {
+        const int m0 = mstart + i0;
+        float cv[4], nv[4];
+        if (m0 >= 0 && m0 + 3 < T) {
+            float4 nz;
+            if (noise_row) nz = __ldg(reinterpret_cast<const float4*>(noise_row + m0));   // m0 % 4 == 0
+            else nz = normals4(seed, utt, (uint32_t)(m0 >> 2));
+            nv[0] = nz.x; nv[1] = nz.y; nv[2] = nz.z; nv[3] = nz.w;
+#pragma unroll
+            for (int e = 0; e < 4; ++e) cv[e] = comb_at(fpar, P, fP, m0 + e);
+        } else {
+#pragma unroll 1
+            for (int e = 0; e < 4; ++e) {
+                int m = m0 + e;
+                bool valid = true;
+                if (m < 0 || m >= T) {
+                    if (reflect) m = (m < 0) ? -m : 2 * (T - 1) - m;
+                    else valid = false;
+                }
+                cv[e] = 0.f; nv[e] = 0.f;
+                if (valid) {
+                    cv[e] = comb_at(fpar, P, fP, m);
+                    if (noise_row) nv[e] = noise_row[m];
+                    else {
+                        const float4 g = normals4(seed, utt, (uint32_t)(m >> 2));
+                        const int l = m & 3;
+                        nv[e] = l == 0 ? g.x : l == 1 ? g.y : l == 2 ? g.z : g.w;
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int e = 0; e < 4; ++e) src[(i0 + e + off) & (kN - 1)] = make_float2(cv[e], nv[e]);
+    }
+}
+
 // shared-memory footprint (bytes): 2 x 17408 (bufA, bufS) + 16384 (src) + 12288 (ring) + 4112 (win)
 // + 1920 (tw2) + 2048 (tw3) = 71568  -> 3 CTAs per SM
 constexpr int kWinLen = kHalf + 4;   // window stored for i in [0, 1024]; win[i] = win[2048 - i]
@@ -228,64 +299,17 @@ __global__ void __launch_bounds__(kThreads, 3) superfast_kernel(SfParams p) {
     const int b = blockIdx.y;
     const int nF = p.nF, P = p.P, T = nF * P;
     const int h0 = blockIdx.x * p.G, h1 = min(h0 + p.G, nF);
-    const float fP = (float)P;
-    const bool reflect = T > kHalf;                              // pad_mode (:672-675)
     const float4* fpar = p.frame_par + (size_t)b * nF;
     const float* noise_row = p.noise_in ? p.noise_in + (size_t)b * T : nullptr;
     const unsigned long long utt = (unsigned long long)(p.utt_off + b);
 
     // ---- one-time tables ----
-    for (int i = tid; i <= kHalf; i += kThreads) winh[i] = 0.5f - 0.5f * cospif((float)i * (2.0f / kN));
-    for (int i = tid; i < 15 * 16; i += kThreads) {
-        const int r = i / 16 + 1, k = i % 16;
-        float sn, cs; sincospif(-2.0f * (float)(r * k) / 256.0f, &sn, &cs);
-        tw2[i] = make_float2(cs, sn);
-    }
-    for (int i = tid; i < 256; i += kThreads) {
-        float sn, cs; sincospif(-2.0f * (float)i / 2048.0f, &sn, &cs);
-        tw3[i] = make_float2(cs, sn);
-    }
+    init_tables(winh, tw2, tw3, tid);
     for (int i = tid; i < kRingHops * kHop; i += kThreads) ring[i] = 0.f;
     __syncthreads();
-    auto win_at = [&](int i) { return winh[i <= kHalf ? i : kN - i]; };
-
-    // source samples of absolute positions [mstart + i_lo, mstart + i_hi) -> src ring slots (i + off) & 2047
+    auto win_at = [&](int i) { return win_of(winh, i); };
     auto fill_src = [&](int mstart, int off, int i_lo, int i_hi) {
-#pragma unroll 1
-        for (int i0 = i_lo + (tid << 2); i0 < i_hi; i0 += kThreads << 2) {
-            const int m0 = mstart + i0;
-            float cv[4], nv[4];
-            if (m0 >= 0 && m0 + 3 < T) {
-                float4 nz;
-                if (noise_row) nz = __ldg(reinterpret_cast<const float4*>(noise_row + m0));   // m0 % 4 == 0
-                else nz = normals4(p.seed, utt, (uint32_t)(m0 >> 2));
-                nv[0] = nz.x; nv[1] = nz.y; nv[2] = nz.z; nv[3] = nz.w;
-#pragma unroll
-                for (int e = 0; e < 4; ++e) cv[e] = comb_at(fpar, P, fP, m0 + e);
-            } else {
-#pragma unroll 1
-                for (int e = 0; e < 4; ++e) {
-                    int m = m0 + e;
-                    bool valid = true;
-                    if (m < 0 || m >= T) {
-                        if (reflect) m = (m < 0) ? -m : 2 * (T - 1) - m;
-                        else valid = false;
-                    }
-                    cv[e] = 0.f; nv[e] = 0.f;
-                    if (valid) {
-                        cv[e] = comb_at(fpar, P, fP, m);
-                        if (noise_row) nv[e] = noise_row[m];
-                        else {
-                            const float4 g = normals4(p.seed, utt, (uint32_t)(m >> 2));
-                            const int l = m & 3;
-                            nv[e] = l == 0 ? g.x : l == 1 ? g.y : l == 2 ? g.z : g.w;
-                        }
-                    }
-                }
-            }
-#pragma unroll
-            for (int e = 0; e < 4; ++e) src[(i0 + e + off) & (kN - 1)] = make_float2(cv[e], nv[e]);
-        }
+        fill_source(src, fpar, noise_row, p.seed, utt, T, P, mstart, off, i_lo, i_hi, tid);
     };
 
     const int qs = max(h0 - 1, 0), qe = min(h1 + 1, nF);
@@ -394,19 +418,167 @@ __global__ void __launch_bounds__(kThreads, 3) superfast_kernel(SfParams p) {
                 const int n = h * P + i4;
                 float v[4] = {acc.x, acc.y, acc.z, acc.w};
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    float env = 0.f;     // OLA(win^2) over the frames that exist
-#pragma unroll
-                    for (int d = -1; d <= 2; ++d) {
-                        const int qq = h + d;
-                        if (qq >= 0 && qq <= nF) { const float w = win_at(i4 + e - d * kHop + kHalf); env = fmaf(w, w, env); }
-                    }
-                    v[e] = __fdiv_rn(v[e], env);
-                }
+                for (int e = 0; e < 4; ++e) v[e] = __fdiv_rn(v[e], ola_env(winh, h, i4 + e, nF));
                 b2d::st_global_v4(p.out + (size_t)b * T + n, make_float4(v[0], v[1], v[2], v[3]));
             }
         }
         __syncthreads();
+    }
+}
+
+// ---- backward: gradients of the four controls from g = dL/dsignal ---------------------------------------
+// Adjoint of trim, envelope division, OLA and synthesis window:  u_q[i] = w[i] g[n] / env(n), n = qP - 1024 + i
+// (0 outside [0, T));  adjoint of irfft:  G_q[k] = (c_k / N) FFT(u_q)[k], c_0 = c_1024 = 1, else 2.
+// With the recomputed filtered spectra Yh = X exp(m_h + j pi p_h), Yn = Z exp(m_n + j pi p_n) / 128 of frame q:
+//   dL/dm = Re(conj(G) Y),   dL/dp = pi Im(G conj(Y))          (row min(q, nF-1); frame nF folds into row nF-1)
+// Frames are independent (no overlap-add), so a CTA walks a run of frame PAIRS (2m, 2m+1) with no halo:
+//  * per pair ONE complex FFT of u_2m + j u_2m+1, split by conjugate symmetry into both frames' G;
+//  * per frame ONE complex FFT of w (comb + j noise), split the same way (the forward's source, recomputed from
+//    the frame parameters and the noise stream, so nothing but the controls is kept for the backward);
+//  * g / env is kept in a ring indexed by sample position, like the source; each pair adds 1024 new samples.
+// The pairing does not depend on the chunking, and every gradient row is written once by the CTA that owns it,
+// so the result is bit-identical for every chunk size, batch split and utterance_offset shard.
+struct SfBwdParams {
+    const float4* frame_par;   // [B, nF]
+    const float* c_hm; const float* c_hp; const float* c_nm; const float* c_np;
+    long long ctrl_stride;
+    const float* noise_in;     // [B, T] or nullptr
+    const float* grad;         // [B, T]
+    float* g_hm; float* g_hp; float* g_nm; float* g_np;
+    long long grad_stride;
+    int nF, P, GP;             // GP: frame pairs per CTA
+    unsigned long long seed;
+    long long utt_off;
+};
+
+constexpr int kGRing = 4096;   // g / env ring (a pair reads 2560 consecutive samples)
+// 2 x 17408 (bufA, bufS) + 16384 (src) + 16384 (g ring) + 4112 (win) + 1920 (tw2) + 2048 (tw3) = 75664 -> 3 CTAs/SM
+constexpr size_t kBwdSmemBytes = (size_t)2 * kPadN * sizeof(float2) + (size_t)kN * sizeof(float2) +
+                                 (size_t)kGRing * sizeof(float) + (size_t)kWinLen * sizeof(float) +
+                                 (size_t)(15 * 16 + 256) * sizeof(float2);
+
+template <bool PK>
+__global__ void __launch_bounds__(kThreads, 3) superfast_backward_kernel(SfBwdParams p) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float2* bufA = reinterpret_cast<float2*>(smem_raw);          // [kPadN] source frame / its spectrum
+    float2* bufS = bufA + kPadN;                                 // [kPadN] u pair / its spectrum
+    float2* src = bufS + kPadN;                                  // [kN]   un-windowed (comb, noise), ring-indexed
+    float2* tw2 = src + kN;
+    float2* tw3 = tw2 + 15 * 16;
+    float* gring = reinterpret_cast<float*>(tw3 + 256);          // [4096] g / env by sample position
+    float* winh = gring + kGRing;                                // [1025]
+
+    const int tid = threadIdx.x;
+    const int b = blockIdx.y;
+    const int nF = p.nF, P = p.P, T = nF * P;
+    const int n_pairs = (nF + 1) / 2;                            // pairs of gradient rows 0..nF-1
+    const int m0 = blockIdx.x * p.GP, m1 = min(m0 + p.GP, n_pairs);
+    const int qe = (m1 == n_pairs) ? nF + 1 : 2 * m1;            // frames [2 m0, qe): the last CTA adds frame nF
+    const float4* fpar = p.frame_par + (size_t)b * nF;
+    const float* noise_row = p.noise_in ? p.noise_in + (size_t)b * T : nullptr;
+    const float* grow = p.grad + (size_t)b * T;
+    const unsigned long long utt = (unsigned long long)(p.utt_off + b);
+
+    init_tables(winh, tw2, tw3, tid);
+    __syncthreads();
+
+    float keep[4][9];      // row nF-1 of frame nF-1, added to frame nF's in registers before the one store
+    int off = 0;
+    bool primed = false;
+    for (int qa = 2 * m0; qa < qe; qa += 2) {
+        const int qb = qa + 1;
+        const bool has_b = qb < qe;
+        const int n0 = qa * P - kHalf;                           // first sample of frame qa
+        // ---- g / env of samples [n0, n0 + 2560): the first pair fills all, later pairs the 1024 new ones ----
+        for (int n = (qa == 2 * m0 ? n0 : n0 + 3 * kHop) + tid; n < n0 + 5 * kHop; n += kThreads) {
+            float v = 0.f;
+            if (n >= 0 && n < T) v = __fdiv_rn(__ldg(grow + n), ola_env(winh, n >> 9, n & (kHop - 1), nF));
+            gring[n & (kGRing - 1)] = v;
+        }
+        __syncthreads();
+        // ---- u pair = w (g/env)[frame qa] + j w (g/env)[frame qb] ----
+#pragma unroll 4
+        for (int i = tid; i < kN; i += kThreads) {
+            const float w = win_of(winh, i);
+            const float ua = w * gring[(n0 + i) & (kGRing - 1)];
+            const float ub = has_b ? w * gring[(n0 + kHop + i) & (kGRing - 1)] : 0.f;
+            bufS[padi(i)] = make_float2(ua, ub);
+        }
+        __syncthreads();
+        fft2048<PK>(bufS, tw2, tw3, tid);
+#pragma unroll 1
+        for (int which = 0; which < 2; ++which) {
+            if (which == 1 && !has_b) break;
+            const int q = which ? qb : qa;
+            const int mstart = q * P - kHalf;
+            if (!primed) { fill_source(src, fpar, noise_row, p.seed, utt, T, P, mstart, off, 0, kN, tid); primed = true; }
+            else { off = (off + kHop) & (kN - 1); fill_source(src, fpar, noise_row, p.seed, utt, T, P, mstart, off, kN - kHop, kN, tid); }
+            __syncthreads();
+#pragma unroll 4
+            for (int i = tid; i < kN; i += kThreads) {
+                const float2 v = src[(i + off) & (kN - 1)];
+                const float w = win_of(winh, i);
+                bufA[padi(i)] = make_float2(w * v.x, w * v.y);
+            }
+            const int qc = min(q, nF - 1);
+            const size_t crow = ((size_t)b * nF + qc) * p.ctrl_stride;
+            float chm[9], chp[9], cnm[9], cnp[9];
+#pragma unroll
+            for (int it = 0; it < 8; ++it) {
+                const size_t o = crow + tid + it * kThreads;
+                chm[it] = __ldg(p.c_hm + o); chp[it] = __ldg(p.c_hp + o);
+                cnm[it] = __ldg(p.c_nm + o); cnp[it] = __ldg(p.c_np + o);
+            }
+            chm[8] = chp[8] = cnm[8] = cnp[8] = 0.f;
+            if (tid == 0) {
+                chm[8] = __ldg(p.c_hm + crow + kHalf); chp[8] = __ldg(p.c_hp + crow + kHalf);
+                cnm[8] = __ldg(p.c_nm + crow + kHalf); cnp[8] = __ldg(p.c_np + crow + kHalf);
+            }
+            __syncthreads();
+            fft2048<PK>(bufA, tw2, tw3, tid);
+            const size_t grow_out = ((size_t)b * nF + qc) * p.grad_stride;
+#pragma unroll
+            for (int it = 0; it < 9; ++it) {
+                const int bin = (it < 8) ? tid + it * kThreads : kHalf;
+                if (it == 8 && tid != 0) break;
+                const int mir = (kN - bin) & (kN - 1);
+                // comb / noise spectra of this frame
+                const float2 za = bufA[padi(bin)];
+                float2 zb = bufA[padi(mir)];
+                zb.y = -zb.y;
+                const float2 X = make_float2(0.5f * (za.x + zb.x), 0.5f * (za.y + zb.y));
+                const float2 d = csub(za, zb);
+                const float2 Nz = make_float2(0.5f * d.y, -0.5f * d.x);
+                // this frame's half of the u-pair spectrum, scaled by c_k / N
+                const float2 sa = bufS[padi(bin)];
+                float2 sb = bufS[padi(mir)];
+                sb.y = -sb.y;
+                const float c = (bin == 0 || bin == kHalf) ? (1.0f / kN) : (2.0f / kN);
+                float2 G;
+                if (which == 0) G = make_float2(0.5f * c * (sa.x + sb.x), 0.5f * c * (sa.y + sb.y));
+                else G = make_float2(0.5f * c * (sa.y - sb.y), -0.5f * c * (sa.x - sb.x));
+                float sh, ch, sn, cn;
+                __sincosf(B2D_PI_F * chp[it], &sh, &ch);
+                __sincosf(B2D_PI_F * cnp[it], &sn, &cn);
+                const float eh = __expf(chm[it]), en = __expf(cnm[it]) * 0.0078125f;
+                const float2 Yh = cmul(X, make_float2(eh * ch, eh * sh));
+                const float2 Yn = cmul(Nz, make_float2(en * cn, en * sn));
+                float gr[4] = {G.x * Yh.x + G.y * Yh.y, B2D_PI_F * (G.y * Yh.x - G.x * Yh.y),
+                               G.x * Yn.x + G.y * Yn.y, B2D_PI_F * (G.y * Yn.x - G.x * Yn.y)};
+                if (q == nF - 1) {
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) keep[t][it] = gr[t];
+                    continue;
+                }
+                if (q == nF) {
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) gr[t] = keep[t][it] + gr[t];
+                }
+                const size_t o = grow_out + bin;
+                p.g_hm[o] = gr[0]; p.g_hp[o] = gr[1]; p.g_nm[o] = gr[2]; p.g_np[o] = gr[3];
+            }
+            __syncthreads();
+        }
     }
 }
 
@@ -464,5 +636,49 @@ extern "C" int b2d_superfast_synth(const void* workspace, const float* c_harmoni
     const int rc = b2d::g_fft_packed.load(std::memory_order_relaxed) ? go(superfast_kernel<true>) : go(superfast_kernel<false>);
     if (rc) return rc;
     return b2d::check_launch("superfast_synth");
+}
+
+extern "C" int b2d_superfast_backward(const void* workspace, const float* c_harmonic_magnitude,
+                                      const float* c_harmonic_phase, const float* c_noise_magnitude,
+                                      const float* c_noise_phase, int64_t ctrl_stride, const float* noise_in,
+                                      uint64_t seed, int64_t utterance_offset, const float* grad_signal, int B,
+                                      int n_frames, int block, int win_length, float* g_harmonic_magnitude,
+                                      float* g_harmonic_phase, float* g_noise_magnitude, float* g_noise_phase,
+                                      int64_t grad_stride, void* stream) {
+    if (!workspace || !c_harmonic_magnitude || !c_harmonic_phase || !c_noise_magnitude || !c_noise_phase ||
+        !grad_signal || !g_harmonic_magnitude || !g_harmonic_phase || !g_noise_magnitude || !g_noise_phase)
+        return b2d::fail(B2D_ERR_NULL, "superfast_backward: null pointer");
+    if (B <= 0 || n_frames <= 0 || block <= 0 || ctrl_stride < win_length / 2 + 1 || grad_stride < win_length / 2 + 1)
+        return b2d::fail(B2D_ERR_SHAPE, "superfast_backward: bad shape");
+    if (win_length != kN || block != 512)
+        return b2d::fail(B2D_ERR_UNSUPPORTED, "superfast_backward: only win_length=2048 / block_size=512 is implemented "
+                         "(got %d / %d)", win_length, block);
+    if (B > 65535) return b2d::fail(B2D_ERR_UNSUPPORTED, "superfast_backward: batch %d > 65535", B);
+    if (!b2d::aligned16(workspace) || (noise_in && !b2d::aligned16(noise_in)))
+        return b2d::fail(B2D_ERR_ALIGN, "superfast_backward: noise_in / workspace must be 16-byte aligned");
+    SfBwdParams p;
+    p.frame_par = static_cast<const float4*>(workspace);
+    p.c_hm = c_harmonic_magnitude; p.c_hp = c_harmonic_phase; p.c_nm = c_noise_magnitude; p.c_np = c_noise_phase;
+    p.ctrl_stride = ctrl_stride; p.noise_in = noise_in; p.grad = grad_signal;
+    p.g_hm = g_harmonic_magnitude; p.g_hp = g_harmonic_phase; p.g_nm = g_noise_magnitude; p.g_np = g_noise_phase;
+    p.grad_stride = grad_stride;
+    p.nF = n_frames; p.P = block;
+    // frame pairs per CTA: no halo to amortise, so shrink the chunk until there are >= ~4 CTAs per SM
+    const int n_pairs = (n_frames + 1) / 2;
+    int GP = 16;
+    while (GP > 2 && (long long)B * ((n_pairs + GP - 1) / GP) < 4 * 148) GP -= 2;
+    p.GP = GP;
+    p.seed = seed; p.utt_off = utterance_offset;
+    auto go = [&](auto kern) -> int {
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmemBytes);
+        if (e != cudaSuccess) return b2d::fail((int)e, "superfast_backward: smem attr: %s", cudaGetErrorString(e));
+        cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        kern<<<dim3((n_pairs + GP - 1) / GP, B), kThreads, kBwdSmemBytes, (cudaStream_t)stream>>>(p);
+        return 0;
+    };
+    const int rc = b2d::g_fft_packed.load(std::memory_order_relaxed) ? go(superfast_backward_kernel<true>)
+                                                                      : go(superfast_backward_kernel<false>);
+    if (rc) return rc;
+    return b2d::check_launch("superfast_backward");
 }
 #endif  // B2D_HOST_EMU

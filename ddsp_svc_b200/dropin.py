@@ -70,12 +70,37 @@ def load_model(model_path, device="cuda"):
     return model, args
 
 
-def patch_reference():
+def _trainable_superfast(unit2ctrl_cls):
+    """CombSubSuperFast whose control network is the reference's own Unit2Control (eager torch, differentiable, the
+    same parameter tree, so checkpoints stay interchangeable); the synthesis runs on the B200 kernels with their
+    fused backward."""
+
+    class CombSubSuperFast(vocoder.CombSubSuperFast):
+        def __init__(self, sampling_rate, block_size, win_length, n_unit=256, n_spk=1, use_pitch_aug=False,
+                     pcmer_norm=False):
+            u2c = unit2ctrl_cls(n_unit, n_spk, vocoder.CombSubSuperFast.split_map(win_length),
+                                use_pitch_aug=use_pitch_aug, use_naive_v2=True, use_conv_stack=True)
+            super().__init__(sampling_rate, block_size, win_length, n_unit=n_unit, n_spk=n_spk,
+                             use_pitch_aug=use_pitch_aug, pcmer_norm=pcmer_norm, unit2ctrl=u2c)
+
+    return CombSubSuperFast
+
+
+def patch_reference(training=False):
     """Swap the synthesizer classes inside the (importable) reference package.  Returns the dict
     of original classes so a caller can restore them; its keys say what was patched.  If the enhancer stack
     (nsf_hifigan.models) cannot be imported, only the synthesizers are patched and the reason is returned under
-    ``"_not_patched"`` -- any other failure propagates."""
+    ``"_not_patched"`` -- any other failure propagates.
+
+    ``training=True`` (for the reference's train.py and the reflow / diffusion training that calls it through
+    ``ddsp_loss``): rebinds only ``ddsp.vocoder.CombSubSuperFast``, to a class that builds the reference's own
+    ``ddsp.unit2control.Unit2Control``; every other class keeps the reference's (they have no backward here)."""
     import ddsp.vocoder as ref_vocoder          # the reference checkout must be on sys.path
+    if training:
+        import ddsp.unit2control as ref_u2c
+        saved = {"CombSubSuperFast": ref_vocoder.CombSubSuperFast}
+        ref_vocoder.CombSubSuperFast = _trainable_superfast(ref_u2c.Unit2Control)
+        return saved
     names = ("Sins", "CombSub", "CombSubSuperFast", "CombSubFast")
     saved = {name: getattr(ref_vocoder, name) for name in names}
     for name in names:

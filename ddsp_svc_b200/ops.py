@@ -362,6 +362,40 @@ def superfast_synth(ws, c_hm, c_hp, c_nm, c_np, block, win_length, noise_in=None
     return signal
 
 
+def superfast_backward(ws, c_hm, c_hp, c_nm, c_np, grad_signal, block, win_length, noise_in=None, seed=0,
+                       utterance_offset=0):
+    """dL/dcontrols of superfast_synth given grad_signal = dL/dsignal [B, T]; the other arguments are those of the
+    forward call (same noise_in, or the same seed and utterance_offset).  Returns the four gradients
+    [B, n_frames, win_length/2+1], views of one dense [B, n_frames, 4 (win_length/2+1)] tensor."""
+    if c_hm.dim() != 3:
+        raise ValueError("controls must be [B, n_frames, win_length/2+1]")
+    B, nF = c_hm.shape[0], c_hm.shape[1]
+    if not isinstance(ws, torch.Tensor) or not ws.is_cuda or ws.dtype != torch.uint8 or \
+            ws.numel() < _lib.lib().b2d_superfast_workspace_bytes(B, nF):
+        raise ValueError("ws must be the workspace superfast_scan returned for the same (B, n_frames) = (%d, %d)" % (B, nF))
+    (hm, hp, nm, npz), stride = _same_stride([("harmonic_magnitude", c_hm), ("harmonic_phase", c_hp),
+                                              ("noise_magnitude", c_nm), ("noise_phase", c_np)], B, nF)
+    C = win_length // 2 + 1
+    if hm.shape[2] != C:
+        raise ValueError("controls must have win_length/2+1 = %d bins" % C)
+    T = nF * block
+    _need_cuda_f32("grad_signal", grad_signal)
+    if tuple(grad_signal.shape) != (B, T):
+        raise ValueError("grad_signal must be [B, n_frames*block] = [%d, %d], got %s" % (B, T, tuple(grad_signal.shape)))
+    grad_signal = grad_signal.contiguous()
+    if noise_in is not None:
+        noise_in = _noise_rows(noise_in, B, T)
+    dense = torch.empty(B, nF, 4 * C, dtype=torch.float32, device=hm.device)
+    grads = torch.split(dense, C, dim=-1)
+    rc = _lib.lib().b2d_superfast_backward(ws.data_ptr(), hm.data_ptr(), hp.data_ptr(), nm.data_ptr(), npz.data_ptr(),
+                                           stride, _ptr(noise_in), int(seed), int(utterance_offset),
+                                           grad_signal.data_ptr(), B, nF, int(block), int(win_length),
+                                           *(g.data_ptr() for g in grads), dense.stride(1), _stream())
+    _lib.check(rc, "b2d_superfast_backward")
+    _count(1)
+    return grads
+
+
 def source_module(f0, upp, sampling_rate, dim, rand_ini, linear_weight, linear_bias, sine_amp=0.1, noise_std=0.003,
                   voiced_threshold=0.0, noise_in=None, seed=0, utterance_offset=0):
     """SineGen + tanh(Linear(dim -> 1)) fused: f0 [B, nF] -> [B, nF*upp, 1]  (nsf_hifigan/models.py:201-204)."""

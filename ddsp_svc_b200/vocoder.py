@@ -130,10 +130,36 @@ class CombSub(_SynthBase):
         return signal, hidden, (harmonic, noise_out)
 
 
+class _SuperFastSynth(torch.autograd.Function):
+    """superfast_synth with a backward for the four controls (the fused kernel of b2d_superfast_backward).  The
+    forward is the inference kernel unchanged; the backward recomputes the source from the scan workspace and the
+    noise from noise_in or (seed, utterance_offset), so nothing but the controls is kept alive."""
+
+    @staticmethod
+    def forward(ctx, ws, hm, hp, nm, np_, block, win, noise, seed, utterance_offset):
+        signal = ops.superfast_synth(ws, hm, hp, nm, np_, block, win, noise_in=noise, seed=seed,
+                                     utterance_offset=utterance_offset)
+        ctx.save_for_backward(ws, hm, hp, nm, np_, noise)
+        ctx.args = (block, win, seed, utterance_offset)
+        return signal
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_signal):
+        ws, hm, hp, nm, np_, noise = ctx.saved_tensors
+        block, win, seed, utterance_offset = ctx.args
+        grads = ops.superfast_backward(ws, hm, hp, nm, np_, grad_signal, block, win, noise_in=noise, seed=seed,
+                                       utterance_offset=utterance_offset)
+        return (None,) + tuple(grads) + (None,) * 5
+
+
 class CombSubSuperFast(_SynthBase):
     """Combtooth subtractive synthesiser (STFT-domain filtering; what configs/combsub.yaml
     selects) -- reference ddsp/vocoder.py:613-710.  Returns (signal, hidden, (signal, signal))
-    with the same tensor three times, like the reference."""
+    with the same tensor three times, like the reference.
+
+    Trainable: when grad is enabled and a control requires grad, the signal is differentiable with respect to the
+    four controls (fused backward kernel); gradients to f0 and to explicit noise are not provided."""
 
     def __init__(self, sampling_rate, block_size, win_length, n_unit=256, n_spk=1, use_pitch_aug=False,
                  pcmer_norm=False, unit2ctrl=None):
@@ -144,14 +170,14 @@ class CombSubSuperFast(_SynthBase):
         self.register_buffer("block_size", torch.tensor(block_size))
         self.register_buffer("win_length", torch.tensor(win_length))
         self.register_buffer("window", torch.hann_window(win_length))
-        split_map = {
-            "harmonic_magnitude": win_length // 2 + 1,
-            "harmonic_phase": win_length // 2 + 1,
-            "noise_magnitude": win_length // 2 + 1,
-            "noise_phase": win_length // 2 + 1,
-        }
         self.unit2ctrl = unit2ctrl if unit2ctrl is not None else _reference_unit2ctrl(
-            n_unit, n_spk, split_map, use_pitch_aug=use_pitch_aug, use_naive_v2=True, use_conv_stack=True)
+            n_unit, n_spk, self.split_map(win_length), use_pitch_aug=use_pitch_aug, use_naive_v2=True,
+            use_conv_stack=True)
+
+    @staticmethod
+    def split_map(win_length):
+        n = int(win_length) // 2 + 1
+        return {"harmonic_magnitude": n, "harmonic_phase": n, "noise_magnitude": n, "noise_phase": n}
 
     def _scalars(self):
         c = self.__dict__.get("_scalar_cache")
@@ -167,11 +193,18 @@ class CombSubSuperFast(_SynthBase):
         ws, phase_frames = ops.superfast_scan(f0_frames, block, sr)
         ctrls, hidden = self.unit2ctrl(units_frames, f0_frames, phase_frames, volume_frames, spk_id=spk_id,
                                        spk_mix_dict=spk_mix_dict, aug_shift=aug_shift)
-        self._forward_only(ctrls)
-        signal = ops.superfast_synth(ws, ctrls["harmonic_magnitude"], ctrls["harmonic_phase"],
-                                     ctrls["noise_magnitude"], ctrls["noise_phase"], block, win, noise_in=noise,
-                                     seed=0 if noise is not None else _host_seed(),
-                                     utterance_offset=utterance_offset, signal_out=signal_out)
+        c = [ctrls[k] for k in ("harmonic_magnitude", "harmonic_phase", "noise_magnitude", "noise_phase")]
+        seed = 0 if noise is not None else _host_seed()
+        if torch.is_grad_enabled() and any(v.requires_grad for v in c):
+            if f0_frames.requires_grad or (noise is not None and noise.requires_grad):
+                raise NotImplementedError("CombSubSuperFast on B200 differentiates with respect to the four controls "
+                                          "only; detach f0_frames and noise")
+            if signal_out is not None:
+                raise ValueError("signal_out cannot be combined with a differentiable forward")
+            signal = _SuperFastSynth.apply(ws, *c, block, win, noise, seed, utterance_offset)
+        else:
+            signal = ops.superfast_synth(ws, *c, block, win, noise_in=noise, seed=seed,
+                                         utterance_offset=utterance_offset, signal_out=signal_out)
         return signal, hidden, (signal, signal)
 
 

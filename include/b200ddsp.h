@@ -213,6 +213,19 @@ int    b2d_superfast_synth(const void* workspace, const float* c_harmonic_magnit
                            const float* c_noise_phase, int64_t ctrl_stride, const float* noise_in,
                            uint64_t seed, int64_t utterance_offset, int B, int n_frames, int block,
                            int win_length, float* signal, void* stream);
+/* Backward of b2d_superfast_synth with respect to its four controls.  grad_signal [B, n_frames*block]
+ * = dL/dsignal (contiguous); the same workspace, controls, noise_in / seed / utterance_offset as the
+ * forward call (the source and the in-kernel noise are recomputed, not stored).  Writes
+ * dL/dcontrol [B, n_frames, win_length/2+1] for each control with frame stride grad_stride (one dense
+ * [B, n_frames, 4 (win_length/2+1)] buffer can hold all four); row n_frames-1 includes the repeated
+ * last frame.  Every element is written once; the result does not depend on how the batch is split. */
+int    b2d_superfast_backward(const void* workspace, const float* c_harmonic_magnitude,
+                              const float* c_harmonic_phase, const float* c_noise_magnitude,
+                              const float* c_noise_phase, int64_t ctrl_stride, const float* noise_in,
+                              uint64_t seed, int64_t utterance_offset, const float* grad_signal, int B,
+                              int n_frames, int block, int win_length, float* g_harmonic_magnitude,
+                              float* g_harmonic_phase, float* g_noise_magnitude, float* g_noise_phase,
+                              int64_t grad_stride, void* stream);
 
 /* SineGen fused with the tail of SourceModuleHnNSF.   replaces nsf_hifigan/models.py:201-204
  * (sine_merge = tanh(l_linear(sine_wavs))) on top of b2d_sinegen: merged [B, n_frames*upp] =
